@@ -27,6 +27,12 @@ Output: ONE JSON line (rank 0).
              value / e2e / roofline / cpu_baseline.
 `--impl reference` times the reference's CPU path alone (same metric / config strings, so the
 driver can divide).
+
+`--dump-outputs DIR` writes the hits of the last timed step of the main workload as
+DIR/items.npy (float64 row ordinals), DIR/scores.npy (float32) and DIR/counts.npy (float64);
+entries past a query's count are -1 / NaN.  Inputs are seeded, so two builds run with the same
+arguments can be compared output for output.  Above 64 MB a fixed, seeded sample of the queries
+is written, their indices in DIR/query_index.npy.  Apart from DIR the bench writes no files.
 """
 
 from __future__ import annotations
@@ -44,6 +50,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the tree may be read-only; keep the bench from writing __pycache__ into it
 
 WORKLOADS = {
     # name: rows, dim, storage, batch, k, min_score
@@ -86,7 +93,35 @@ def parse_args():
     p.add_argument("--no-parity", action="store_true", help="skip the blocked-oracle check of the final step")
     p.add_argument("--sustain-seconds", type=float, default=2.0, help="0 disables the sustained roofline run")
     p.add_argument("--cpu-queries", type=int, default=8, help="timed single-query lookups of the cpu_baseline leg")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="write the hits of the last timed step as DIR/<name>.npy (see the module docstring)")
+    args = p.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        p.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "b200":
+        p.error("--dump-outputs writes the GPU path's hits; it needs --impl b200")
+    return args
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(dump_dir, items, scores, counts):
+    """Hits of one step (device tensors [B, k], [B, k], [B]) -> dump_dir/{items,scores,counts}.npy."""
+    counts = counts.cpu().numpy().astype(np.int64)
+    items = items.cpu().numpy().astype(np.float64)      # row ordinals < 2**53: exact
+    scores = scores.cpu().numpy().astype(np.float32)
+    past = np.arange(items.shape[1])[None, :] >= counts[:, None]
+    items[past], scores[past] = -1.0, np.nan
+    arrays = {"items": items, "scores": scores, "counts": counts.astype(np.float64)}
+    per_query = sum(a[0].nbytes for a in arrays.values())
+    if per_query * len(counts) > DUMP_LIMIT_BYTES:
+        keep = np.sort(np.random.default_rng(SEED).choice(len(counts), DUMP_LIMIT_BYTES // per_query, replace=False))
+        arrays = {name: a[keep] for name, a in arrays.items()}
+        arrays["query_index"] = keep.astype(np.float64)
+    os.makedirs(dump_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(dump_dir, name + ".npy"), a)
 
 
 def metric_string(w):
@@ -428,7 +463,8 @@ class Bench:
             self.dist.destroy_process_group()
 
 
-def measure(bn: Bench, name, w, steps, warmup, *, force=None, sustain_s=0.0, parity=True, cpu=True, cpu_queries=8):
+def measure(bn: Bench, name, w, steps, warmup, *, force=None, sustain_s=0.0, parity=True, cpu=True, cpu_queries=8,
+            dump_dir=None):
     """One workload on the GPUs of this run -> the result dict (rank 0) or None (other ranks)."""
     import typeagent_py_b200 as tab
     from typeagent_py_b200.sharded import ShardedVectorBase, shard_bounds
@@ -515,6 +551,8 @@ def measure(bn: Bench, name, w, steps, warmup, *, force=None, sustain_s=0.0, par
         m = got.value
         return {"main": list(arr[0][:m]), "sample": list(arr[1][:m]), "aux": list(arr[2][:m]), "search_total": list(arr[3][:m])}
 
+    last_hits = [None]   # (items, scores, counts) of the latest timed step
+
     def timed_resident(n_steps):
         """EXACTLY n_steps steps, CUDA events on the launching stream; returns total ms (this rank)."""
         total = 0.0
@@ -523,7 +561,7 @@ def measure(bn: Bench, name, w, steps, warmup, *, force=None, sustain_s=0.0, par
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             e0.record()
             for i in range(n_steps):
-                step_resident()
+                last_hits[0] = step_resident()
                 if (i & 7) == 7:
                     finish_resident()      # at most 8 (sharded) / 64 searches may be outstanding
             finish_resident()
@@ -535,7 +573,7 @@ def measure(bn: Bench, name, w, steps, warmup, *, force=None, sustain_s=0.0, par
             bn.barrier()
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             e0.record()
-            step_resident()
+            last_hits[0] = step_resident()
             finish_resident()
             e1.record()
             bn.barrier()
@@ -551,6 +589,8 @@ def measure(bn: Bench, name, w, steps, warmup, *, force=None, sustain_s=0.0, par
 
     sampler = ClockSampler(bn.local_rank) if rank == 0 else None
     ms_resident = bn.max_over_ranks(timed_resident(steps))
+    # later steps reuse the output buffers: copy the last timed step's hits (stream-ordered, untimed)
+    dumped = tuple(t.clone() for t in last_hits[0]) if dump_dir and rank == 0 else None
     hist = history(steps)                       # the SAME pass as ms_resident
     # rank-to-rank spread of the local search (a sharded step ends when the SLOWEST rank has published)
     per_rank = None
@@ -621,6 +661,8 @@ def measure(bn: Bench, name, w, steps, warmup, *, force=None, sustain_s=0.0, par
     parity_checked, parity_note = False, "skipped"
     if parity:
         parity_checked, parity_note = check_parity(bn, corpus, lo, qn, items, scores, counts, k, w["min_score"], storage)
+    if dumped is not None:
+        dump_outputs(dump_dir, *dumped)
 
     del corpus, base, sharded
     torch.cuda.empty_cache()
@@ -738,14 +780,15 @@ def run_b200(args, w):
     bn = Bench(args)
     force = None if args.path == "auto" else args.path
     out = measure(bn, args.workload, w, args.steps, args.warmup, force=force, sustain_s=args.sustain_seconds,
-                  parity=not args.no_parity, cpu=not args.no_cpu_baseline, cpu_queries=args.cpu_queries)
+                  parity=not args.no_parity, cpu=not args.no_cpu_baseline, cpu_queries=args.cpu_queries,
+                  dump_dir=args.dump_outputs)
     # the other BASELINE configs ride along so that the driver's records carry them
     secondary = {}
     if not args.no_secondary and args.workload == "c3" and args.rows is None:
         names = ["c1", "c2", "c5"] if bn.world == 1 else (["c4"] if bn.world == 8 else [])
         for name in names:
             sw = dict(WORKLOADS[name])
-            res = measure(bn, name, sw, steps=max(args.steps, 10), warmup=max(args.warmup, 3), sustain_s=0.0,
+            res = measure(bn, name, sw, steps=args.steps, warmup=args.warmup, sustain_s=0.0,
                           parity=not args.no_parity, cpu=not args.no_cpu_baseline, cpu_queries=args.cpu_queries)
             if res is not None:
                 keep = ("metric", "value", "unit", "ms_per_step", "path", "e2e", "roofline", "cpu_baseline",

@@ -19,8 +19,10 @@ EPISODE53_FILE = os.path.join(HERE, "episode53_excerpt.npy")
 GOLDEN_FILE = os.path.join(HERE, "golden_cases.json")
 
 # rows of tests/testdata/Episode_53_AdrianTchaikovsky_index_embeddings.bin kept in the
-# excerpt: the first 300 related-term rows and all 106 message-chunk rows (1188..1293)
-EPISODE53_ROWS = list(range(300)) + list(range(1188, 1294))
+# excerpt (150 x 1536 float32, under 1 MB): the first 100 related-term rows and the first 50 of
+# the 106 message-chunk rows (1188..1293)
+EPISODE53_TERMS = 100
+EPISODE53_ROWS = list(range(EPISODE53_TERMS)) + list(range(1188, 1238))
 
 
 def unit_rows(rng, n, d):
@@ -52,7 +54,7 @@ def episode53():
     # queries: a few term rows and a few message rows, slightly perturbed so that the
     # best hit is not a trivial exact duplicate with score 1.0 only
     rng = np.random.default_rng(53)
-    picks = [0, 7, 123, 299, 300, 350, 405]
+    picks = [0, 7, 61, 99, 100, 125, 149]
     q = v[picks] + 0.05 * unit_rows(rng, len(picks), v.shape[1])
     q /= np.linalg.norm(q, axis=1, keepdims=True)
     return v, q.astype(np.float32)
@@ -62,7 +64,11 @@ def _mod3(i: int) -> bool:
     return i % 3 == 0
 
 
-PREDICATES = {"mod3": _mod3}
+def _odd(i: int) -> bool:
+    return i % 2 == 1
+
+
+PREDICATES = {"mod3": _mod3, "odd": _odd}
 
 
 # Each case: name, how to build (vectors, queries), and the lookups to record.
@@ -104,7 +110,8 @@ CASES: list[dict] = [
          lookups=[("lookup", dict(max_hits=50, min_score=0.85)),
                   ("lookup", dict(max_hits=10, min_score=0.7)),
                   ("lookup", dict(max_hits=25, min_score=0.0)),
-                  ("subset", dict(subset=("range", 300, 406), max_hits=25, min_score=0.7))]),
+                  ("subset", dict(subset=("range", EPISODE53_TERMS, len(EPISODE53_ROWS)), max_hits=25,
+                                  min_score=0.7))]),
 ]
 
 
@@ -127,3 +134,61 @@ def build_subset(spec) -> list[int]:
     if tag == "range":
         return list(range(spec[1], spec[2]))
     raise ValueError(tag)
+
+
+def reference_lookup(base, q, kind, kw):
+    """One recorded lookup through a reference ``VectorBase``."""
+    kw = dict(kw)
+    if kind == "lookup":
+        return base.fuzzy_lookup_embedding(q, **kw)
+    if kind == "subset":
+        return base.fuzzy_lookup_embedding_in_subset(q, build_subset(kw.pop("subset")), **kw)
+    if kind == "predicate":
+        return base.fuzzy_lookup_embedding(q, predicate=PREDICATES[kw.pop("predicate")], **kw)
+    raise ValueError(kind)
+
+
+def as_record(hits) -> dict:
+    return {"items": [h.item for h in hits], "scores": [h.score for h in hits]}
+
+
+# Randomised shapes (corpus size and dimension drawn from the seed).  Some lookups return half
+# the corpus, so their recorded outputs are kept as arrays in RANDOM_FILE (see random_record).
+RANDOM_SEEDS = [1, 2, 3]
+RANDOM_FILE = os.path.join(HERE, "random_cases.npz")
+
+
+def random_key(seed, query, lookup) -> str:
+    return f"s{seed}_q{query}_l{lookup}"
+
+
+def random_record(arrays, seed, query, lookup) -> dict:
+    key = random_key(seed, query, lookup)
+    return {"items": arrays[key + "_items"].tolist(), "scores": arrays[key + "_scores"].tolist()}
+
+
+def random_case(seed):
+    """(vectors, queries, lookups): lookups[i] is the list of (kind, kwargs) run for query i."""
+    from oracle.vectorbase_oracle import make_corpus
+
+    rng = np.random.default_rng(seed)
+    n, d = int(rng.integers(50, 3000)), int(rng.choice([3, 64, 384, 769]))
+    v, q = make_corpus(n, d, seed, n_queries=3)
+    lookups = []
+    for _ in q:
+        per = [("lookup", dict(max_hits=k, min_score=ms))
+               for k, ms in ((10, 0.0), (None, None), (5, 0.5), (n + 5, 0.49), (0, 0.52))]
+        subset = rng.choice(n, size=min(n, 40), replace=True).tolist()
+        per.append(("subset", dict(subset=("list", subset), max_hits=7, min_score=0.3)))
+        per.append(("predicate", dict(predicate="odd", max_hits=6, min_score=0.4)))
+        lookups.append(per)
+    return v, q, lookups
+
+
+# Lookups of the Episode-53 excerpt stored as an embedding-file pair: (which part, max_hits,
+# min_score), recorded per query under GOLDEN["embedding_file_pair"].
+EMBEDDING_FILE_LOOKUPS = [("related", 50, 0.85), ("messages", 10, 0.7), ("messages", 25, 0.0)]
+
+
+def embedding_file_key(part, max_hits, min_score) -> str:
+    return f"{part}/{max_hits}/{min_score}"

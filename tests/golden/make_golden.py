@@ -6,9 +6,10 @@ Run in the build container only (needs /root/reference):
     python tests/golden/make_golden.py
 
 Writes ``golden_cases.json`` (reference outputs: items + float32 scores as Python
-floats, which round-trip exactly through JSON) and ``episode53_excerpt.npy`` (406 of
+floats, which round-trip exactly through JSON) and ``episode53_excerpt.npy`` (150 of
 the 1294 real embedding rows of the reference's Episode-53 test fixture).  Also records
-the reference's own known-answer tests as literal cases.
+the reference's own known-answer tests as literal cases, and the outputs of the randomised
+cases as arrays in ``random_cases.npz``.
 """
 
 from __future__ import annotations
@@ -37,26 +38,37 @@ def main() -> None:
     for case in C.CASES:
         vectors, queries = C.build_inputs(case)
         base = make_reference_vectorbase(vectors)
-        recorded = []
-        for kind, kw in case["lookups"]:
-            per_query = []
-            for q in queries:
-                if kind == "lookup":
-                    hits = base.fuzzy_lookup_embedding(q, **kw)
-                elif kind == "subset":
-                    kw2 = dict(kw)
-                    subset = C.build_subset(kw2.pop("subset"))
-                    hits = base.fuzzy_lookup_embedding_in_subset(q, subset, **kw2)
-                elif kind == "predicate":
-                    kw2 = dict(kw)
-                    pred = C.PREDICATES[kw2.pop("predicate")]
-                    hits = base.fuzzy_lookup_embedding(q, predicate=pred, **kw2)
-                else:
-                    raise ValueError(kind)
-                per_query.append({"items": [h.item for h in hits], "scores": [h.score for h in hits]})
-            recorded.append(per_query)
+        recorded = [[C.as_record(C.reference_lookup(base, q, kind, kw)) for q in queries]
+                    for kind, kw in case["lookups"]]
         out["cases"][case["name"]] = recorded
         print(f"{case['name']}: {len(recorded)} lookups x {len(queries)} queries")
+
+    arrays = {}
+    for seed in C.RANDOM_SEEDS:
+        vectors, queries, lookups = C.random_case(seed)
+        base = make_reference_vectorbase(vectors)
+        for qi, (q, per) in enumerate(zip(queries, lookups)):
+            for li, (kind, kw) in enumerate(per):
+                hits = C.reference_lookup(base, q, kind, kw)
+                key = C.random_key(seed, qi, li)
+                arrays[key + "_items"] = np.array([h.item for h in hits], np.int32)
+                arrays[key + "_scores"] = np.array([h.score for h in hits], np.float32)   # exact: float32 scores
+    np.savez_compressed(C.RANDOM_FILE, **arrays)
+
+    # Episode-53 excerpt split as an embedding-file pair (related terms, message chunks)
+    ep, epq = C.episode53()
+    parts = {"related": make_reference_vectorbase(ep[:C.EPISODE53_TERMS]),
+             "messages": make_reference_vectorbase(ep[C.EPISODE53_TERMS:])}
+    out["embedding_file_pair"] = {
+        C.embedding_file_key(part, k, ms): [C.as_record(parts[part].fuzzy_lookup_embedding(q, max_hits=k, min_score=ms))
+                                            for q in epq]
+        for part, k, ms in C.EMBEDDING_FILE_LOOKUPS}
+
+    # state of a VectorBase after the calls of test_oracle_class_matches_reference_class_api
+    base = make_reference_vectorbase()
+    base.add_embedding(None, [0.7, 0.8, 0.9])
+    base.add_embeddings(None, np.array([[0.1, 0.2, 0.3], [0.4, 0.5, 0.6]], np.float32))
+    out["class_api_serialized"] = base.serialize().tolist()
 
     # The reference's own known-answer test (tests/test_vectorbase.py:239-252).
     base = make_reference_vectorbase()

@@ -138,9 +138,9 @@ def _assert_terms_match(got, want, tie=2e-6):
 
 
 def _vocabularies():
-    ep, epq = C.episode53()                      # real data: 406 x 1536 (terms 0..299, message chunks 300..405)
-    yield "episode53", ep[:300], epq, 50, 0.85
-    yield "episode53-lowfloor", ep[:300], epq, 10, 0.0
+    ep, epq = C.episode53()                      # real data: 150 x 1536 (terms 0..99, message chunks 100..149)
+    yield "episode53", ep[:C.EPISODE53_TERMS], epq, 50, 0.85
+    yield "episode53-lowfloor", ep[:C.EPISODE53_TERMS], epq, 10, 0.0
     v, q = O.make_corpus(6000, 384, seed=61, n_queries=64)   # >= 4096 rows, >= 16 queries: tensor cores
     yield "synthetic-6000x384", v, q, 5, 0.0
 
@@ -210,32 +210,33 @@ def test_reference_built_indexes_return_reference_hits_after_install(name, vecto
         assert mem._vectorbase.last_timing()["path"] in ("scan", "mma_split")
 
 
-@needs_reference
 @pytest.mark.gpu
 def test_embedding_file_pair_loads_into_a_search(tmp_path):
     """The reference's on-disk layout (knowpro/serialization.py:83-98, :183-222): <prefix>_embeddings.bin
-    + <prefix>_data.json -> formats.load_embedding_file -> GPU lookups equal to the reference's."""
+    + <prefix>_data.json -> formats.load_embedding_file -> GPU lookups equal to the reference's
+    (its outputs recorded by tests/golden/make_golden.py)."""
     from typeagent_py_b200 import formats
 
+    with open(C.GOLDEN_FILE) as f:
+        want = json.load(f)["embedding_file_pair"]
     ep, epq = C.episode53()
-    related, messages = ep[:300], ep[300:]
+    related, messages = ep[:C.EPISODE53_TERMS], ep[C.EPISODE53_TERMS:]
     prefix = str(tmp_path / "Episode_53_excerpt_index")
     formats.write_embedding_file(prefix, related, messages)
     raw = np.fromfile(prefix + "_embeddings.bin", dtype=np.float32).reshape(-1, ep.shape[1])   # podcasts/podcast.py:147-168
     np.testing.assert_array_equal(raw, ep)
     settings = tab.TextEmbeddingIndexSettings(O.FakeEmbeddingModel())
     rel_base, msg_base = formats.load_embedding_file(prefix, settings)
-    assert len(rel_base) == 300 and len(msg_base) == 106
-    ref_rel = ref_loader.make_reference_vectorbase(related)
-    ref_msg = ref_loader.make_reference_vectorbase(messages)
-    for q in epq:
-        for base, ref, k, ms in ((rel_base, ref_rel, 50, 0.85), (msg_base, ref_msg, 10, 0.7), (msg_base, ref_msg, 25, 0.0)):
-            got = base.fuzzy_lookup_embedding(q, k, ms)
-            want = ref.fuzzy_lookup_embedding(q, max_hits=k, min_score=ms)
-            assert_hits_match(got, want, min_score=ms, what="embedding file -> search")   # order up to float32 ties
+    assert len(rel_base) == len(related) and len(msg_base) == len(messages)
+    bases = {"related": rel_base, "messages": msg_base}
+    for qi, q in enumerate(epq):
+        for part, k, ms in C.EMBEDDING_FILE_LOOKUPS:
+            got = bases[part].fuzzy_lookup_embedding(q, k, ms)
+            assert_hits_match(got, want[C.embedding_file_key(part, k, ms)][qi], min_score=ms,
+                              what="embedding file -> search")   # order up to float32 ties
     # SQLite BLOB layout (storage/sqlite/schema.py:193-212) through embeddings_from_blobs
     blobs = [row.tobytes() for row in messages]
     again = tab.VectorBase(settings)
     again.deserialize(formats.embeddings_from_blobs(blobs))
     assert_hits_match(again.fuzzy_lookup_embedding(epq[4], 10, 0.7),
-                      ref_msg.fuzzy_lookup_embedding(epq[4], max_hits=10, min_score=0.7), min_score=0.7)
+                      want[C.embedding_file_key("messages", 10, 0.7)][4], min_score=0.7)

@@ -3,7 +3,8 @@
 1. committed golden vectors generated from the unmodified reference
    (tests/golden/make_golden.py);
 2. the reference's own known-answer tests (tests/test_vectorbase.py:239-252, :209-236);
-3. when /root/reference is mounted (build container), the live reference on fresh inputs.
+3. the reference on randomised shapes and through its class API: recorded outputs, and the live
+   reference as well where its sources can be loaded (``oracle/ref_loader.py``).
 """
 
 from __future__ import annotations
@@ -108,38 +109,33 @@ def test_fake_embedding_known_values():
         O.fake_text_embedding("", 3)
 
 
-@pytest.mark.skipif(not reference_available(), reason="reference not mounted (GPU box)")
-@pytest.mark.parametrize("seed", [1, 2, 3])
+@pytest.mark.parametrize("seed", C.RANDOM_SEEDS)
 def test_oracle_matches_live_reference(seed):
-    rng = np.random.default_rng(seed)
-    n, d = int(rng.integers(50, 3000)), int(rng.choice([3, 64, 384, 769]))
-    v, q = O.make_corpus(n, d, seed, n_queries=3)
-    ref = make_reference_vectorbase(v)
-    for qq in q:
-        for k, ms in ((10, 0.0), (None, None), (5, 0.5), (n + 5, 0.49), (0, 0.52)):
-            want = ref.fuzzy_lookup_embedding(qq, max_hits=k, min_score=ms)
-            got = O.lookup(v, qq, k, ms)
-            assert [h.item for h in got] == [h.item for h in want]
-            assert [h.score for h in got] == [h.score for h in want]
-        subset = rng.choice(n, size=min(n, 40), replace=True).tolist()
-        want = ref.fuzzy_lookup_embedding_in_subset(qq, subset, 7, 0.3)
-        got = O.lookup_in_subset(v, qq, subset, 7, 0.3)
-        assert [(h.item, h.score) for h in got] == [(h.item, h.score) for h in want]
-        want = ref.fuzzy_lookup_embedding(qq, 6, 0.4, predicate=lambda i: i % 2 == 1)
-        got = O.lookup(v, qq, 6, 0.4, predicate=lambda i: i % 2 == 1)
-        assert [(h.item, h.score) for h in got] == [(h.item, h.score) for h in want]
+    """Randomised shapes: the oracle against the reference's recorded outputs and, where the
+    reference sources can be loaded, against the live reference bit for bit."""
+    v, q, lookups = C.random_case(seed)
+    ref = make_reference_vectorbase(v) if reference_available() else None
+    with np.load(C.RANDOM_FILE) as arrays:
+        for qi, (qq, per) in enumerate(zip(q, lookups)):
+            for li, (kind, kw) in enumerate(per):
+                got = run_oracle_lookup(v, qq, kind, kw)
+                assert_hits_match(got, C.random_record(arrays, seed, qi, li), score_tol=2e-6,
+                                  min_score=kw.get("min_score"), what=f"seed {seed}/q{qi}/{kind}/{kw}")
+                if ref is not None:
+                    want = C.reference_lookup(ref, qq, kind, kw)
+                    assert [(h.item, h.score) for h in got] == [(h.item, h.score) for h in want]
 
 
-@pytest.mark.skipif(not reference_available(), reason="reference not mounted (GPU box)")
 def test_oracle_class_matches_reference_class_api():
-    """Same state after the same calls; same errors (tests/test_vectorbase.py:72-102,255-277)."""
+    """Same state after the same calls as the reference (recorded, and live where its sources can
+    be loaded); same errors (tests/test_vectorbase.py:72-102,255-277)."""
     from types import SimpleNamespace
 
     model = O.FakeEmbeddingModel()
     mine = O.OracleVectorBase(SimpleNamespace(embedding_model=model, min_score=0.85, max_matches=None))
-    ref = make_reference_vectorbase()
+    ref = make_reference_vectorbase() if reference_available() else None
     rows = np.array([[0.1, 0.2, 0.3], [0.4, 0.5, 0.6]], np.float32)
-    for b in (mine, ref):
+    for b in (mine, ref) if ref is not None else (mine,):
         assert len(b) == 0 and bool(b) is True
         b.add_embedding(None, [0.7, 0.8, 0.9])
         b.add_embeddings(None, rows)
@@ -150,6 +146,10 @@ def test_oracle_class_matches_reference_class_api():
         with pytest.raises(IndexError):
             b.get_embedding_at(3)
         assert b.serialize_embedding_at(9) is None
-    np.testing.assert_array_equal(mine.serialize(), ref.serialize())
-    mine.clear(), ref.clear()
-    assert mine.serialize().shape == ref.serialize().shape == (0, 3)
+    np.testing.assert_array_equal(mine.serialize(), np.array(GOLDEN["class_api_serialized"], np.float32))
+    if ref is not None:
+        np.testing.assert_array_equal(mine.serialize(), ref.serialize())
+        ref.clear()
+        assert ref.serialize().shape == (0, 3)
+    mine.clear()
+    assert mine.serialize().shape == (0, 3)
